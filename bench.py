@@ -15,6 +15,11 @@ lp_clusterer.cc:89-109) on the synthetic input, the timed region of the referenc
            stand-in) or, when that library is absent, the oracle port, on a bounded sample
 
 ``--impl reference`` times only the CPU reference arm on the same workload definition.
+
+``--dump-outputs DIR`` writes what the last timed step computed (the arrays a caller of the timed path receives)
+to DIR/<name>.npy; the inputs are generated from fixed seeds, so two builds can be compared output for output.
+The LP random draws are seeded per call (like the reference's), so the last step's result depends on
+--warmup + --steps: compare runs made with the same arguments.
 """
 from __future__ import annotations
 
@@ -86,6 +91,31 @@ def generate(name, device):
         raise ValueError(kind)
     xadj, adj, _ = G.rearrange_by_degree_buckets_torch(xadj, adj, remove_isolated=True)
     return xadj, adj, k
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as <out_dir>/<name>.npy: float32 where each value is exact in it (|x| <= 2^24), float64
+    otherwise. When the total exceeds DUMP_BUDGET_BYTES, every array larger than its share of the budget is cut to
+    a sample of positions drawn with a fixed seed (the same positions for the same length in every run); the
+    positions go to <name>_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        out[name] = a.astype(np.float32 if a.size == 0 or np.abs(a).max() <= (1 << 24) else np.float64)
+    if sum(a.nbytes for a in out.values()) > DUMP_BUDGET_BYTES:
+        share = DUMP_BUDGET_BYTES // len(out)
+        for name in list(out):
+            a = out[name]
+            if a.nbytes > share:
+                idx = np.sort(np.random.default_rng(0).choice(a.size, share // (a.itemsize + 8), replace=False))
+                out[name] = a[idx]
+                out[name + "_index"] = idx.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -228,14 +258,20 @@ def contraction_mode(args, handle, g_host, n, m, k, mcw, dev, local_rank):
     torch.cuda.synchronize()
     sampler.mark_begin()
     tot_ms, launches, last = 0.0, 0, None
-    for _ in range(args.steps):
+    for step in range(args.steps):
         cg = KC.contract_on_handle(handle, None)
         tot_ms += cg.stats.device_ms
         launches += cg.stats.kernel_launches
         last = (cg.stats.c_n, cg.stats.c_m, cg.stats.cut_edges, cg.stats.sort_bits)
-        cg.close()
+        if args.dump_outputs is None or step + 1 < args.steps:
+            cg.close()
     torch.cuda.synchronize()
     sampler.mark_end()
+    if args.dump_outputs is not None:  # the coarse graph of the last timed step
+        c = cg.get()
+        dump_outputs(args.dump_outputs, {"c_xadj": c.xadj, "c_adjncy": c.adjncy, "c_vwgt": c.vwgt,
+                                         "c_adjwgt": c.adjwgt, "mapping": cg.mapping()})
+        cg.close()
     clocks = sampler.stop()
     value = m * args.steps / (tot_ms * 1e-3)
     c_n, c_m, cut, bits = last
@@ -302,7 +338,14 @@ def main():
     ap.add_argument("--mode", default="clustering", choices=["clustering", "refinement", "contraction"],
                     help="refinement: one LabelPropagationRefiner.refine call on a hashed k-way partition (N=1 only); "
                          "contraction: contract_clustering of the LP clustering (SURVEY §8f-1, N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, <= 64 MB "
+                         "in all): clustering; partition + block_weights; c_xadj, c_adjncy, c_vwgt, c_adjwgt, mapping")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.workload is None:
         args.workload = "rmat22" if args.gpus <= 1 else "rmat24"
 
@@ -391,11 +434,13 @@ def main():
         mbw = ctx.partition.max_block_weights()
 
     sharded_moved = []  # per-round move counts of the last sharded step (identical on every rank)
+    block_weights = [None]  # returned by the last refinement step
 
     def run_resident():
         if refine_handle is not None:
             refine_handle.upload_partition(part0)
-            return refine_handle.refine(k, mbw, None)[2]
+            _, block_weights[0], st = refine_handle.refine(k, mbw, None)
+            return st
         return handle.cluster(mcw, fetch=False)[1]
 
     def barrier():
@@ -431,6 +476,12 @@ def main():
         last = st
     barrier()
     sampler.mark_end()
+    if args.dump_outputs is not None and rank == 0:  # the labels the last timed step left on the device
+        if refine_handle is not None:
+            dump_outputs(args.dump_outputs, {"partition": refine_handle.download_labels(),
+                                             "block_weights": block_weights[0]})
+        else:
+            dump_outputs(args.dump_outputs, {"clustering": handle.download_labels()})
     # ---- breakdown steps (outside the timed region): per-tier CUDA events, tiers serialised ----------------
     BSTEPS = 2
     (refine_handle or handle).set_timing(True)

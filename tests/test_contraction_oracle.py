@@ -1,17 +1,17 @@
 """Pins the contraction oracle (oracle/contraction_oracle.py): golden vectors produced by the unmodified
-reference (tests/golden/contract_*.npz), the reference's own known-answer tests
-(tests/shm/coarsening/cluster_contraction_test.cc), the live reference when it is built, and
-size-independent properties."""
+reference (tests/golden/contract_*.npz, tests/golden/live_reference.npz), the reference's own known-answer
+tests (tests/shm/coarsening/cluster_contraction_test.cc) and size-independent properties."""
+import hashlib
 import os
 
 import numpy as np
 import pytest
 
 from kaminpar_b200 import graph as G
-from oracle import bindings as B
 from oracle import contraction_oracle as CO
 from tests import helpers as H
 
+LIVE = os.path.join(H.GOLDEN, "live_reference.npz")
 CASES = ["rgg2d_k4", "rgg16_w", "walshaw_k16", "walshaw_unsorted", "rmat13_w", "grid12", "road60", "star30000"]
 
 
@@ -74,16 +74,34 @@ def test_reference_kats():
     assert o["c_adjwgt"].sum() == 12 and {(11, 22), (22, 33), (33, 44)} <= weighted_endpoints(o)
 
 
-@pytest.mark.skipif(not B.have_reference(), reason="oracle/_ref not built (authoring container only)")
+def live_graphs():
+    return [G.rmat(12, 8, 3), G.grid3d(9), G.random_weights(G.rgg2d(3000, 1), 5, max_vwgt=3, max_adjwgt=5), H.big_star(5000)]
+
+
+def live_clusterings(g, rng):
+    return (rng.integers(0, g.n, g.n).astype(np.uint32), np.arange(g.n, dtype=np.uint32),
+            (np.arange(g.n) // 7 * 7).astype(np.uint32), np.zeros(g.n, np.uint32))
+
+
+def digest(o):
+    """sha256 of a canonical contraction result (the fixture stores the reference's as this fingerprint)."""
+    h = hashlib.sha256(np.int64(o["c_n"]).tobytes())
+    for key, dtype in (("c_xadj", np.uint32), ("c_adjncy", np.uint32), ("c_vwgt", np.int32), ("c_adjwgt", np.int32),
+                       ("mapping", np.uint32)):
+        h.update(np.ascontiguousarray(o[key], dtype).tobytes())
+    return h.hexdigest()
+
+
 @pytest.mark.parametrize("algorithm", [0, 1, 2])
 def test_oracle_matches_live_reference(algorithm):
+    """The oracle == the reference's BUFFERED (0), UNBUFFERED (1) and UNBUFFERED_NAIVE (2) contraction after
+    canonicalisation; the reference's results are stored by tests/golden/make_live_reference_golden.py."""
+    d = np.load(LIVE)
+    want = zip(d[f"contract_a{algorithm}_c_n"], d[f"contract_a{algorithm}_c_m"], d[f"contract_a{algorithm}_sha256"])
     rng = np.random.default_rng(algorithm)
-    graphs = [G.rmat(12, 8, 3), G.grid3d(9), G.random_weights(G.rgg2d(3000, 1), 5, max_vwgt=3, max_adjwgt=5), H.big_star(5000)]
-    for g in graphs:
-        for cl in (rng.integers(0, g.n, g.n).astype(np.uint32), np.arange(g.n, dtype=np.uint32),
-                   (np.arange(g.n) // 7 * 7).astype(np.uint32), np.zeros(g.n, np.uint32)):
-            r = B.ref_contract(g, cl, algorithm)
-            assert CO.equal(oracle_of(g, cl), CO.canonicalize(**r, clustering=cl))
+    got = [(o["c_n"], len(o["c_adjncy"]), digest(o)) for g in live_graphs() for o in
+           (oracle_of(g, cl) for cl in live_clusterings(g, rng))]
+    assert got == [(int(c_n), int(c_m), str(h)) for c_n, c_m, h in want]
 
 
 def test_properties():
@@ -113,21 +131,24 @@ def test_empty_graph():
     assert o["c_n"] == 0 and len(o["c_xadj"]) == 1
 
 
-@pytest.mark.skipif(not B.have_reference(), reason="oracle/_ref not built (authoring container only)")
-def test_oracle_matches_live_reference_random_multigraphs():
-    """Random small graphs with parallel edges, self-loops and weights, random clusterings: the oracle ==
-    the unmodified reference (default algorithm) after canonicalisation."""
-    from hypothesis import given, settings
-    from hypothesis import strategies as st
-
-    @settings(max_examples=40, deadline=None)
-    @given(st.integers(1, 40), st.integers(0, 120), st.integers(0, 2**31 - 1))
-    def run(n, m_und, seed):
+def multigraph_cases():
+    """Random small graphs with parallel edges, self-loops and weights, and random clusterings (seeded)."""
+    draw = np.random.default_rng(2)
+    params = [(1, 0, 0), (1, 3, 1), (40, 0, 2), (40, 120, 3)]
+    params += [(int(draw.integers(1, 41)), int(draw.integers(0, 121)), int(draw.integers(0, 2**31 - 1))) for _ in range(36)]
+    for n, m_und, seed in params:
         rng = np.random.default_rng(seed)
         edges = [(int(a), int(b)) for a, b in rng.integers(0, n, (m_und, 2))]
         g = H.from_edges(n, edges, vwgt=rng.integers(1, 5, n), ew=rng.integers(1, 6, m_und).tolist())
-        cl = rng.integers(0, n, n).astype(np.uint32)
-        r = B.ref_contract(g, cl, 1)
-        assert CO.equal(oracle_of(g, cl), CO.canonicalize(**r, clustering=cl))
+        yield g, rng.integers(0, n, n).astype(np.uint32)
 
-    run()
+
+def test_oracle_matches_live_reference_random_multigraphs():
+    """The oracle == the unmodified reference (default algorithm, raw results stored by
+    tests/golden/make_live_reference_golden.py) after canonicalisation."""
+    d = np.load(LIVE)
+    cases = list(multigraph_cases())
+    assert len(cases) == len(d["multigraph_c_n"])
+    for i, (g, cl) in enumerate(cases):
+        r = {k: d[f"multigraph{i}_{k}"] for k in ("c_xadj", "c_adjncy", "c_vwgt", "c_adjwgt", "mapping")}
+        assert CO.equal(oracle_of(g, cl), CO.canonicalize(int(d["multigraph_c_n"][i]), **r, clustering=cl))

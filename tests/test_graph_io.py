@@ -1,5 +1,6 @@
 """Graph IO (SURVEY §8f-3): METIS text and ParHIP binary readers / writers, partition files -- checked against the
-reference's own sample files where /root/reference is available (authoring container) and by round trips."""
+reference's own sample files (misc/rgg2d*, stored gzip-compressed under tests/golden/) and by round trips."""
+import gzip
 import os
 
 import numpy as np
@@ -9,22 +10,24 @@ from kaminpar_b200.graph import (CSRGraph, random_weights, read_metis, read_parh
                                  write_parhip, write_partition)
 from tests import helpers as H
 
-REF_MISC = "/root/reference/misc"
+
+def sample_file(fname, tmp_path):
+    """The reference's sample file `fname`, unpacked from tests/golden/<fname>.gz into tmp_path."""
+    path = str(tmp_path / fname)
+    with gzip.open(os.path.join(H.GOLDEN, fname + ".gz"), "rb") as src, open(path, "wb") as dst:
+        dst.write(src.read())
+    return path
 
 
 @pytest.mark.parametrize("fname", ["rgg2d-32bit.parhip", "rgg2d-64bit.parhip"])
-def test_parhip_reader_on_the_references_sample_files(fname):
-    path = os.path.join(REF_MISC, fname)
-    if not os.path.exists(path):
-        pytest.skip("reference sample files not available on this box")
-    g = read_parhip(path)
+def test_parhip_reader_on_the_references_sample_files(fname, tmp_path):
+    g = read_parhip(sample_file(fname, tmp_path))
     gold = H.load_graph("rgg2d")  # parsed from misc/rgg2d.metis by the reference (tests/golden/make_golden.py)
     assert g.n == 1024 and g.m == 8226  # test_pykaminpar.py:78-92
     assert np.array_equal(g.xadj, gold.xadj) and np.array_equal(g.adjncy, gold.adjncy)
     assert g.vwgt is None and g.adjwgt is None
-    if os.path.exists(os.path.join(REF_MISC, "rgg2d.metis")):
-        m = read_metis(os.path.join(REF_MISC, "rgg2d.metis"))
-        assert np.array_equal(m.xadj, g.xadj) and np.array_equal(m.adjncy, g.adjncy)
+    m = read_metis(sample_file("rgg2d.metis", tmp_path))
+    assert np.array_equal(m.xadj, g.xadj) and np.array_equal(m.adjncy, g.adjncy)
 
 
 @pytest.mark.parametrize("weights", [(0, 0), (5, 0), (0, 7), (4, 9)])
